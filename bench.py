@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — rows/s and achieved HBM GB/s of the scan -> filter -> group-by/aggregate path (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--rows R] [--config c2|c2all|c3|c4]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--rows R] [--config c2|c2all|c3|c4] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input (BASELINE.json configs[1] at N = 1):
     1e9 rows, c0/c1 int64 ~U[0,1e6), g int32 ~U[0,1e4):  SELECT g, SUM(c1), COUNT(*) FROM t WHERE c0 < 500000 GROUP BY g
@@ -483,6 +483,47 @@ def timed_steps(runner, steps, warmup, torch, dist, sampler=None):
     return rs, float(np.mean(step_ms)), float(np.mean(scan_ms)), t_begin, t_end
 
 
+DUMP_MAX_BYTES = 60_000_000   # array bytes written by --dump-outputs: under 64 MB with the .npy headers
+
+
+def target_names(sql):
+    """File-name-safe names of the SELECT list: "g, SUM(c1), COUNT(*)" -> ["g", "sum_c1", "count"]."""
+    body = sql[len("SELECT "):sql.index(" FROM ")]
+    names, depth, cur = [], 0, ""
+    for ch in body:
+        depth += (ch == "(") - (ch == ")")
+        if ch == "," and depth == 0:
+            names.append(cur)
+            cur = ""
+        else:
+            cur += ch
+    names.append(cur)
+    return ["_".join("".join(c if c.isalnum() else " " for c in n.lower()).split()) for n in names]
+
+
+def dump_outputs(out_dir, rs, sql, ordered):
+    """Writes what the caller of the timed path received in the last step, one float64 array per target as
+    out_dir/col<i>_<target>.npy (NULLs are the target type's inline sentinel), or for the estimator query its NDV estimate
+    and bitmap.  Rows of a GROUP BY without ORDER BY come in hash-table order, which another build may change, so they
+    are sorted by all columns, keys first: two builds then compare row for row.  Beyond DUMP_MAX_BYTES a fixed, seeded
+    sample of the sorted rows is written."""
+    os.makedirs(out_dir, exist_ok=True)
+    if sql.startswith("ESTIMATOR"):
+        arrays = {"ndv_estimate": np.array([rs.getNDVEstimator()], dtype=np.float64),
+                  "estimator_bitmap": rs.getHostEstimatorBuffer().astype(np.float32)}
+    else:
+        cols = [a for _, _, a in rs.columnarResults()]
+        n = cols[0].size
+        order = np.arange(n) if ordered else np.lexsort(cols[::-1])
+        keep = DUMP_MAX_BYTES // (8 * len(cols))
+        if n > keep:
+            order = order[np.sort(np.random.default_rng(SEED).choice(n, size=keep, replace=False))]
+        arrays = {f"col{i}_{name}": a[order].astype(np.float64) for i, (name, a) in enumerate(zip(target_names(sql), cols))}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return sorted(arrays)
+
+
 def config_block(cfg, rows, torch, steps=3, warmup=1):
     """kernel_ms / ms_per_step / roofline fraction / full-size parity of one more BASELINE configuration (N = 1)."""
     peak, _ = measured_peak()
@@ -522,7 +563,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--force-kernel", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result columns of the last timed step to DIR/<name>.npy "
+                    "(float64, at most 64 MB: a seeded row sample beyond that), so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's result; the reference arm has none")
     # the contract is ONE JSON line on stdout: whatever libraries print there (NCCL's version banner, for one) goes to stderr
     global _JSON_OUT
     sys.stdout.flush()
@@ -566,6 +613,9 @@ def main():
     rs, ms, k_ms, t_begin, t_end = timed_steps(runner, args.steps, args.warmup, torch, dist)
     clocks = sampler.stop(t_begin, t_end)
     sql, bytes_per_row = runner.sql, runner.bytes_per_row
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = dump_outputs(args.dump_outputs, rs, sql, ordered=runner.unit.unit.num_order_entries > 0)
     launches_per_step = rs.stats()["kernel_launches"]
     sort_us = rs.stats()["sort_us"]
     result_rows = rs.rowCount() if not sql.startswith("ESTIMATOR") else rs.getNDVEstimator()
@@ -603,6 +653,8 @@ def main():
         "clocks": clocks,
         "gpu_launches": int(launches_per_step) * args.steps,  # per step: b2q_k_init, the scan / radix passes, b2q_k_materialize (+ NCCL's own)
     }
+    if dumped:
+        out["dumped_outputs"] = dumped
     # the timed result, checked bit for bit against the oracle over the full input of ALL ranks
     if not args.no_parity:
         if rank == 0:

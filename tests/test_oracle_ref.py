@@ -1,7 +1,8 @@
-"""Pins the oracle's hash + probe against the reference's OWN runtime compiled verbatim from /root/reference
-(oracle/_ref/libref_groupby.so = QueryEngine/MurmurHash.cpp + QueryEngine/GroupByRuntime.cpp, see
-oracle/ref_shim.cpp), and against the probe constants recorded in SURVEY.md §8c."""
-import ctypes as C
+"""Pins the oracle's hash + probe against the reference's OWN runtime (QueryEngine/MurmurHash.cpp + QueryEngine/GroupByRuntime.cpp +
+QueryEngine/DecodersImpl.h, see oracle/ref_shim.cpp), and against the probe constants recorded in SURVEY.md §8c.  What the reference's
+runtime answered on the inputs below is stored in tests/golden/ref_runtime.npz (made by tools/ref_runtime_golden.py), so these tests
+need neither the reference's sources nor a build of them."""
+import hashlib
 import os
 
 import numpy as np
@@ -10,7 +11,48 @@ import pytest
 import oracle_lib
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_SO = os.path.join(ROOT, "oracle", "_ref", "libref_groupby.so")
+GOLDEN = os.path.join(ROOT, "tests", "golden", "ref_runtime.npz")
+
+GGV_CASES = [(8, 97, 60), (8, 64, 64), (4, 101, 80), (8, 16, 40)]     # (key_width, entry_count, nkeys)
+FAST_CASES = [(5, 0, 0), (17, 3, 0), (40, 10, 2)]                       # (key, min, bucket)
+DECODED_COLUMNS = [("dd", "days"), ("dd16", "days"), ("ts", "fixed"), ("s8", "unsigned"), ("s16", "unsigned")]
+DAY_QUERIES = ["SELECT dt, COUNT(*) FROM s WHERE dt > 1555286410 GROUP BY dt;", "SELECT dd, COUNT(*) FROM s WHERE dd >= 1555372801 GROUP BY dd;"]
+JOIN_SQL = "SELECT COUNT(*), SUM(d.big) FROM t JOIN d ON t.fk32 = d.id32;"
+
+
+def fresh_ggv_buffer(key_width, entry_count, row_size_quad=3):
+    """An empty baseline-hash buffer of rows [key 8][slot][slot]."""
+    b = np.zeros(entry_count * row_size_quad, dtype=np.int64)
+    if key_width == 8:
+        b.reshape(entry_count, row_size_quad)[:, 0] = np.iinfo(np.int64).max
+    else:
+        b.view(np.int32).reshape(entry_count, 2 * row_size_quad)[:, 0] = np.iinfo(np.int32).max
+    return b
+
+
+def decoder_table():
+    import str_tables as stt
+    return stt.str_table(3000, seed=21, frag_rows=700)
+
+
+def day_table():
+    import str_tables as stt
+    return stt.str_table(3000, seed=22, frag_rows=700)
+
+
+def join_tables():
+    import join_tables as jt
+    return jt.dim_table(), jt.fact_table(5000, seed=9, frag_rows=1300)
+
+
+def chunk_digest(*tables_and_columns):
+    """sha256 over the chunks of the given (table, column indices) pairs: ties a stored answer to the exact input it was computed on."""
+    h = hashlib.sha256()
+    for table, cols in tables_and_columns:
+        for f in table.fragments:
+            for c in cols:
+                h.update(np.ascontiguousarray(f.host_cols[c]).tobytes())
+    return h.digest()
 
 
 def test_murmur3_known_answers():
@@ -22,180 +64,105 @@ def test_murmur3_known_answers():
 
 
 @pytest.fixture(scope="module")
-def ref():
-    if not os.path.exists(REF_SO):
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    R = C.CDLL(REF_SO)
-    R.MurmurHash3.restype = C.c_uint32
-    R.MurmurHash3.argtypes = [C.c_void_p, C.c_int, C.c_uint32]
-    R.get_group_value.restype = C.c_void_p
-    R.get_group_value.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]
-    R.get_group_value_fast.restype = C.c_void_p
-    R.get_group_value_fast.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_uint32]
-    return R
+def golden():
+    with np.load(GOLDEN) as z:
+        return {k: z[k] for k in z.files}
 
 
-def test_murmur3_matches_reference(ref):
+def test_murmur3_matches_reference(golden):
     L = oracle_lib.lib()
-    rng = np.random.default_rng(7)
-    data = rng.integers(0, 256, size=64, dtype=np.uint8)
+    data = np.ascontiguousarray(golden["murmur_data"])
     for length in range(0, 33):
-        for seed in (0, 1, 0x9747B28C):
-            assert L.oracle_murmur3(data.ctypes.data, length, seed) == ref.MurmurHash3(data.ctypes.data, length, seed)
-    keys = rng.integers(-2**62, 2**62, size=2000, dtype=np.int64)
+        for j, seed in enumerate(golden["murmur_seeds"]):
+            assert L.oracle_murmur3(data.ctypes.data, length, int(seed)) == golden["murmur_data_hash"][length, j]
+    keys = np.ascontiguousarray(golden["murmur_keys"])
     for i in range(keys.size):
-        p = keys[i:i + 1].ctypes.data
-        assert L.oracle_murmur3(p, 8, 0) == ref.MurmurHash3(p, 8, 0)
+        assert L.oracle_murmur3(keys[i:i + 1].ctypes.data, 8, 0) == golden["murmur_keys_hash"][i]
 
 
-@pytest.mark.parametrize("key_width,entry_count,nkeys", [(8, 97, 60), (8, 64, 64), (4, 101, 80), (8, 16, 40)])
-def test_get_group_value_matches_reference(ref, key_width, entry_count, nkeys):
+@pytest.mark.parametrize("key_width,entry_count,nkeys", GGV_CASES)
+def test_get_group_value_matches_reference(golden, key_width, entry_count, nkeys):
     """Same insert sequence into two tables -> identical slot addresses, identical key placement, and the same
     'table full' answer (NULL) once entry_count distinct keys are in (GroupByRuntime.cpp:25-48)."""
     L = oracle_lib.lib()
-    rng = np.random.default_rng(entry_count)
-    row_size_quad = 3  # [key 8][slot][slot]
-    empty = np.iinfo(np.int64).max if key_width == 8 else None
-    def fresh():
-        b = np.zeros(entry_count * row_size_quad, dtype=np.int64)
-        rows = b.reshape(entry_count, row_size_quad)
-        if key_width == 8:
-            rows[:, 0] = empty
-        else:
-            b.view(np.int32).reshape(entry_count, 2 * row_size_quad)[:, 0] = np.iinfo(np.int32).max
-        return b
-    ours, theirs = fresh(), fresh()
-    keys = rng.integers(1, 50 if entry_count == 16 else 10**6, size=nkeys)
-    keys = np.concatenate([keys, keys[: nkeys // 2]])  # revisit
-    for k in keys:
+    tag = f"ggv_{key_width}_{entry_count}_{nkeys}"
+    keys, want_off = golden[tag + "_keys"], golden[tag + "_off"]
+    ours = fresh_ggv_buffer(key_width, entry_count)
+    for k, r_off in zip(keys, want_off):
         kb = np.zeros(1, dtype=np.int64)
         if key_width == 8:
             kb[0] = k
         else:
             kb.view(np.int32)[0] = k
-        o = L.oracle_get_group_value(ours.ctypes.data, entry_count, kb.ctypes.data, 1, key_width, row_size_quad)
-        r = ref.get_group_value(theirs.ctypes.data, entry_count, kb.ctypes.data, 1, key_width, row_size_quad)
-        r_off = -1 if not r else (r - theirs.ctypes.data) // 8
+        o = L.oracle_get_group_value(ours.ctypes.data, entry_count, kb.ctypes.data, 1, key_width, 3)
         assert o == r_off
         if o >= 0:
             ours[o] += 1
-            theirs[r_off] += 1
-    assert np.array_equal(ours, theirs)
+    assert np.array_equal(ours, golden[tag + "_buf"])
 
 
-def test_get_group_value_fast_reference(ref):
+def test_get_group_value_fast_reference(golden):
     """Perfect-hash direct index: off = (key - min) / bucket * row_size_quad, key written on first touch
     (GroupByRuntime.cpp:194-209) — the formula the oracle's run_fragment and the CUDA kernels use."""
-    row_size_quad, n = 3, 20
-    buf = np.full(n * row_size_quad, np.iinfo(np.int64).max, dtype=np.int64)
-    for key, mn, bucket in [(5, 0, 0), (17, 3, 0), (40, 10, 2)]:
-        r = ref.get_group_value_fast(buf.ctypes.data, key, mn, bucket, row_size_quad)
+    row_size_quad = 3
+    buf = golden["fast_buf"]
+    for (key, mn, bucket), r_off in zip(FAST_CASES, golden["fast_off"]):
         d = key - mn
         if bucket:
             d //= bucket
-        assert (r - buf.ctypes.data) // 8 == d * row_size_quad + 1
+        assert r_off == d * row_size_quad + 1
         assert buf[d * row_size_quad] == key
 
 
-# ---- chunk decoders (QueryEngine/DecodersImpl.h, compiled from the reference) --------------------------------
-def _decoders(ref):
-    for name in ("fixed_width_int_decode", "fixed_width_unsigned_decode"):
-        f = getattr(ref, name)
-        f.restype = C.c_int64
-        f.argtypes = [C.c_void_p, C.c_int32, C.c_int64]
-    ref.fixed_width_small_date_decode.restype = C.c_int64
-    ref.fixed_width_small_date_decode.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int64]
-    return ref
-
-
-def test_chunk_decoders_match_reference(ref):
+def test_chunk_decoders_match_reference(golden):
     """The oracle reads ENCODING FIXED, DICT(8|16) and DATE ENCODING DAYS chunks exactly like the reference's
     decoders: per column, MIN / MAX / COUNT over the values the REFERENCE decodes == the oracle's answer."""
     import sqlmini
     import str_tables as stt
-    from heavydb_b200 import abi
-    _decoders(ref)
-    table = stt.str_table(3000, seed=21, frag_rows=700)
+    table = decoder_table()
     names = stt.STR_NAMES
-    null64 = abi.NULL_BIGINT
-    for col, kind in [("dd", "days"), ("dd16", "days"), ("ts", "fixed"), ("s8", "unsigned"), ("s16", "unsigned")]:
-        c = names.index(col)
-        width = np.dtype(table.physical_dtype(c)).itemsize
-        vals = []
-        for f in table.fragments:
-            a = f.host_cols[c]
-            for pos in range(a.size):
-                if kind == "days":
-                    v = ref.fixed_width_small_date_decode(a.ctypes.data, width, table.physical_null(c), null64, pos)
-                    if v != null64:
-                        vals.append(v)
-                elif kind == "fixed":
-                    v = ref.fixed_width_int_decode(a.ctypes.data, width, pos)
-                    if v != table.physical_null(c):     # codgenAdjustFixedEncNull maps it to the logical NULL
-                        vals.append(v)
-                else:
-                    v = ref.fixed_width_unsigned_decode(a.ctypes.data, width, pos)
-                    if stt.STR_COLS[c][2] or v != table.physical_null(c):
-                        vals.append(v)
+    assert chunk_digest((table, [names.index(c) for c, _ in DECODED_COLUMNS])) == golden["dec_digest"].tobytes()
+    for (col, kind), (mn, mx, count) in zip(DECODED_COLUMNS, golden["dec_min_max_count"].tolist()):
         agg = "COUNT({0})" if kind == "unsigned" else "MIN({0}), MAX({0}), COUNT({0})"
         res = oracle_lib.execute(sqlmini.parse(f"SELECT {agg.format(col)}, COUNT(*) FROM s;", table, names), table).rows()[0]
         if kind == "unsigned":
-            assert res == (len(vals), 3000)
+            assert res == (count, 3000)
         else:
-            assert res == (min(vals), max(vals), len(vals), 3000), col
+            assert res == (mn, mx, count, 3000), col
 
 
-def test_day_bucket_index_matches_reference(ref):
+def test_day_bucket_index_matches_reference(golden):
     """DATE keys: entry = (key - min) / 86400 with min possibly off the day grid (a simple qual narrowed it) — every
     non-empty entry of the oracle's buffer sits where the reference's get_group_value_fast puts its key."""
     import sqlmini
     import str_tables as stt
-    table = stt.str_table(3000, seed=22, frag_rows=700)
-    for sql in ["SELECT dt, COUNT(*) FROM s WHERE dt > 1555286410 GROUP BY dt;", "SELECT dd, COUNT(*) FROM s WHERE dd >= 1555372801 GROUP BY dd;"]:
+    table = day_table()
+    for q, sql in enumerate(DAY_QUERIES):
         res = oracle_lib.execute(sqlmini.parse(sql, table, stt.STR_NAMES), table)
         p = res.plan
         assert p.bucket == 86400 and p.min_val % 86400 != 0 and not p.keyless_hash
         row_quad = p.row_size // 8
+        assert [p.min_val, p.bucket, row_quad, p.entry_count] == golden[f"day{q}_plan"].tolist(), sql
+        ref_off = dict(zip(golden[f"day{q}_keys"].tolist(), golden[f"day{q}_off"].tolist()))
         buf = res.buffer().view(np.int64).reshape(p.entry_count, row_quad)
         seen = 0
         for i in range(p.entry_count):
             key = int(buf[i, 0])
             if key == np.iinfo(np.int64).max:
                 continue
-            scratch = np.full(p.entry_count * row_quad, np.iinfo(np.int64).max, dtype=np.int64)
-            r = ref.get_group_value_fast(scratch.ctypes.data, key, p.min_val, p.bucket, row_quad)
-            assert (r - scratch.ctypes.data) // 8 == i * row_quad + 1, (sql, i, key)
+            assert ref_off.get(key) == i * row_quad + 1, (sql, i, key)
             seen += 1
-        assert seen == res.row_count() > 5
+        assert seen == len(ref_off) == res.row_count() > 5
 
 
-def test_one_to_one_join_table_matches_reference(ref):
+def test_one_to_one_join_table_matches_reference(golden):
     """fill_one_to_one_hashtable + get_hash_slot + hash_join_idx[_nullable] (JoinHashImpl.h, GroupByRuntime.cpp:283-316),
-    the reference's own code, drive a Python join; the oracle's joined aggregates must agree."""
+    the reference's own code, drove a Python join over these tables; the oracle's joined aggregates must agree."""
     import join_tables as jt
     import sqlmini
-    from heavydb_b200 import abi
-    ref.fill_one_to_one_hashtable.restype = C.c_int
-    ref.fill_one_to_one_hashtable.argtypes = [C.c_size_t, C.c_void_p, C.c_int32]
-    ref.get_hash_slot.restype = C.c_void_p
-    ref.get_hash_slot.argtypes = [C.c_void_p, C.c_int64, C.c_int64]
-    ref.hash_join_idx_nullable.restype = C.c_int64
-    ref.hash_join_idx_nullable.argtypes = [C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int64]
-    dim, fact = jt.dim_table(), jt.fact_table(5000, seed=9, frag_rows=1300)
-    ids = dim.fragments[0].host_cols[jt.DIM_NAMES.index("id32")]
-    big = dim.fragments[0].host_cols[jt.DIM_NAMES.index("big")]
-    mn, mx = int(ids.min()), int(ids.max())
-    buff = np.full(mx - mn + 1, -1, dtype=np.int32)
-    for row, k in enumerate(ids):
-        slot = ref.get_hash_slot(buff.ctypes.data, int(k), mn)
-        assert ref.fill_one_to_one_hashtable(row, slot, -1) == 0
-    matches, total = 0, 0
-    for f in fact.fragments:
-        for k in f.host_cols[jt.FACT_NAMES.index("fk32")]:
-            idx = ref.hash_join_idx_nullable(buff.ctypes.data, int(k), mn, mx, abi.NULL_INT)
-            if idx >= 0:
-                matches += 1
-                total += int(big[idx])
-    unit = sqlmini.parse("SELECT COUNT(*), SUM(d.big) FROM t JOIN d ON t.fk32 = d.id32;", fact, jt.FACT_NAMES, inner=(dim, jt.DIM_NAMES))
+    dim, fact = join_tables()
+    assert chunk_digest((dim, range(len(jt.DIM_NAMES))), (fact, range(len(jt.FACT_NAMES)))) == golden["join_digest"].tobytes()
+    matches, total = golden["join_matches_sum"].tolist()
+    unit = sqlmini.parse(JOIN_SQL, fact, jt.FACT_NAMES, inner=(dim, jt.DIM_NAMES))
     assert oracle_lib.execute(unit, fact).rows() == [(matches, total)]
     assert 0 < matches < 5000
