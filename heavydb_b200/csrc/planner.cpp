@@ -679,8 +679,12 @@ class Planner {
         }
       }
       if (!compact) {
+        /* QueryMemoryDescriptor.cpp:826-833 sums the tuples of every input table (query_infos): with a join level, the
+         * inner table's rows count too, although the combined input carries only the outer table's row counts */
         uint64_t tuples = 0;
         for (int f = 0; f < t_.num_fragments; ++f) tuples += static_cast<uint64_t>(t_.fragments[f].num_tuples);
+        if (join_)
+          for (int f = 0; f < inner_->num_fragments; ++f) tuples += static_cast<uint64_t>(inner_->fragments[f].num_tuples);
         width = tuples <= UINT32_MAX ? 4 : 8;
       } else {
         for (int i = 0; i < u_.num_target_exprs; ++i) compact = std::max<int8_t>(compact, static_cast<int8_t>(from_abi(ex(u_.target_exprs[i]).ti).size()));

@@ -691,8 +691,9 @@ void get_keyless_info(const B2QExecUnit& u, const B2QTableInfo& tbl, const std::
 
 constexpr int64_t kMaxBufferSize = int64_t(1) << 30;   /* GroupByAndAggregate.cpp:57 */
 
+/* inner_tuples: the rows of a join level's inner table, which `tbl` (the combined input) does not carry */
 Plan make_plan_single(const B2QExecUnit& u, const B2QTableInfo& tbl, const B2QExecutionOptions& eo,
-                      size_t max_groups_buffer_entry_guess, bool has_cardinality_estimation) {
+                      size_t max_groups_buffer_entry_guess, bool has_cardinality_estimation, uint64_t inner_tuples = 0) {
   if (u.has_union_all || u.has_window_function)
     fail(B2Q_ERR_UNSUPPORTED, "union / window functions are outside this path");
   if (u.has_estimator) {
@@ -912,7 +913,8 @@ Plan make_plan_single(const B2QExecUnit& u, const B2QTableInfo& tbl, const B2QEx
         }
       }
       if (!compact_width) {
-        uint64_t total_tuples = 0;
+        /* :826-830: the tuples of every table in query_infos, the inner table of a join level included */
+        uint64_t total_tuples = inner_tuples;
         for (int f = 0; f < tbl.num_fragments; ++f) total_tuples += tbl.fragments[f].num_tuples;
         min_slot_size = total_tuples <= std::numeric_limits<uint32_t>::max() ? 4 : crt_min_byte_width;
       } else {
@@ -1178,7 +1180,8 @@ void build_joined_input(const B2QExecUnit& u, const B2QTableInfo& outer, JoinedI
   ji.frags.resize(outer.num_fragments);
   for (int f = 0; f < outer.num_fragments; ++f) {
     const B2QFragmentInfo& of = outer.fragments[f];
-    ji.bufs[f].assign(of.col_buffers, of.col_buffers + outer.num_cols);
+    if (of.col_buffers) ji.bufs[f].assign(of.col_buffers, of.col_buffers + outer.num_cols);
+    else ji.bufs[f].assign(static_cast<size_t>(outer.num_cols), nullptr); /* a stats-only fragment: chunk stats, no data */
     ji.stats[f].assign(of.col_stats, of.col_stats + outer.num_cols);
     for (int c = 0; c < n_inner; ++c) {
       ji.bufs[f].push_back(inf ? inf->col_buffers[c] : nullptr);
@@ -1188,7 +1191,7 @@ void build_joined_input(const B2QExecUnit& u, const B2QTableInfo& outer, JoinedI
       if (left) ji.stats[f].back().has_nulls = 1; /* is_outer_join_proj: getLeafColumnRange starts from has_nulls = true (ExpressionRange.cpp:521-525, :642-652) */
     }
     ji.frags[f] = of;
-    ji.frags[f].col_buffers = ji.bufs[f].data();
+    ji.frags[f].col_buffers = of.col_buffers ? ji.bufs[f].data() : nullptr;
     ji.frags[f].col_stats = ji.stats[f].data();
   }
   ji.t = outer;
@@ -1211,8 +1214,10 @@ Plan make_plan(const B2QExecUnit& u, const B2QTableInfo& tbl, const B2QExecution
     fail(B2Q_ERR_UNSUPPORTED, "join keys must be integer columns (dictionary translation is outside this path)");
   if (is_decimal(oti.type) || is_decimal(iti.type)) fail(B2Q_ERR_UNSUPPORTED, "DECIMAL join keys are outside this path");
   if (is_date_in_days(ji.t, ji.outer_col) || is_date_in_days(ji.t, ji.inner_vcol)) fail(B2Q_ERR_UNSUPPORTED, "days-encoded DATE join keys are outside the product path");
-  Plan plan = make_plan_single(ji.u, ji.t, eo, max_groups_buffer_entry_guess, has_cardinality_estimation);
   const B2QTableInfo& inner = *u.inner_table;
+  uint64_t inner_tuples = 0;
+  for (int f = 0; f < inner.num_fragments; ++f) inner_tuples += inner.fragments[f].num_tuples;
+  Plan plan = make_plan_single(ji.u, ji.t, eo, max_groups_buffer_entry_guess, has_cardinality_estimation, inner_tuples);
   Range r; /* getExpressionRange(inner_col): over the inner table alone */
   {
     B2QTableInfo it = inner;
